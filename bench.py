@@ -2,6 +2,7 @@
 """bench.py -- the measurement contract.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload W]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the workload over one batch of synthetic input; rank 0 prints ONE JSON
@@ -19,6 +20,8 @@ inference_input_type=int8 -- int8 images + DEQUANTIZE in the graph, a quarter of
 bytes) or `float32`; at N = 1 the default run reports both (`f32_input`), Bi-RealNet-18 b512 and
 QuickNetLarge b128 (`other_configs`), the same graph on the two older inner products
 (`legacy_paths`), and checks the GPU against the CPU checker on 4 images before it times anything.
+Inputs and weights are seeded, so `--dump-outputs DIR` (the outputs of the last timed step) lets
+two builds be compared output for output.
 
 `--impl reference` times the reference's own CPU kernels (oracle/_ref: its headers compiled by
 oracle/Makefile; LCE ops: bitpack_matrix + Kernel4x2Portable indirect BGEMM + zero-padding
@@ -75,10 +78,42 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip f32_input / other_configs / legacy_paths / parity check")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as "
+                         "DIR/<name>.npy (rank 0; float32, or float64 for integer results)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.workload == "bgemm_sweep"):
+        ap.error("--dump-outputs applies to --impl b200 and the graph / bconv_stack workloads")
     if a.batch <= 0:
         a.batch = DEFAULT_BATCH[a.workload]
     return a
+
+
+DUMP_MAX_ELEMENTS = 1 << 21      # per array: 8 MB as float32; larger outputs are sampled
+DUMP_MAX_BYTES = 64 * 10**6
+
+
+def dump_array(a):
+    """An output as --dump-outputs stores it: float32, or float64 for integers (exact for int32),
+    and, above DUMP_MAX_ELEMENTS, the flattened elements at a fixed seeded set of sorted indices,
+    the same in every run."""
+    a = np.asarray(a)
+    a = a.astype(np.float64 if a.dtype.kind in "iub" or a.dtype == np.float64 else np.float32)
+    if a.size > DUMP_MAX_ELEMENTS:
+        idx = np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False)
+        a = a.reshape(-1)[np.sort(idx)]
+    return a
+
+
+def write_dump(out_dir, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -313,7 +348,7 @@ def main_reference(args):
     if args.workload == "bgemm_sweep":
         emit({"impl": "reference", "unavailable": "bgemm_sweep has no reference arm"})
         return
-    steps = max(1, min(args.steps, 5))          # >= 5 timed steps whenever the caller asks for >= 5
+    steps = args.steps
     warm = min(args.warmup, 1)
     n_img = args.batch                          # the GPU arm's batch: same config on both arms
     r = run_reference(args.workload, n_img, steps, warm, args.input_type)
@@ -479,8 +514,9 @@ def parity_check(model_bytes, input_type, n_img=4):
 
 
 def graph_workload(D, workload, B, input_type, steps, warmup, want_e2e=True, want_profile=True,
-                   model_bytes=None, env=None):
-    """Full `.tflite` graph through the graph host (custom-op registrations)."""
+                   model_bytes=None, env=None, want_outputs=False):
+    """Full `.tflite` graph through the graph host (custom-op registrations). want_outputs: also
+    return the graph outputs of the last timed step (res["outputs"], for --dump-outputs)."""
     torch = D.torch
     from compute_engine_b200 import capi, host as H
     saved = {}
@@ -526,6 +562,8 @@ def graph_workload(D, workload, B, input_type, steps, warmup, want_e2e=True, wan
                "in_bytes": in_bytes, "out_bytes": out_bytes, "fused_nodes_removed": fused,
                "graph_nodes": g.num_nodes(), "arena_bytes": g.arena_bytes(),
                "model_bytes": len(model_bytes), "e2e_ms": None}
+        if want_outputs:
+            res["outputs"] = {f"output{i}": dump_array(g.read(t)) for i, t in enumerate(g.outputs())}
 
         # ---- (2) per-node device times: eager pass with CUDA events on the graph's stream
         if want_profile:
@@ -667,11 +705,18 @@ def stack_workload(args, D):
     sampler = ClockSampler(D.local)
     if D.rank == 0:
         sampler.start()
+    last = []
+
+    def timed_step():
+        last[:] = step(True)
+
     l0 = capi.launch_count()
-    total_ms, w0, w1 = D.timed(lambda: step(True), args.steps, torch.cuda.synchronize)
+    total_ms, w0, w1 = D.timed(timed_step, args.steps, torch.cuda.synchronize)
     launches = capi.launch_count() - l0
     clocks = sampler.stop(w0, w1) if D.rank == 0 else None
     torch.cuda.synchronize()
+    outputs = ({f"stage{s}": dump_array(x.cpu().numpy()) for s, x in enumerate(last)}
+               if args.dump_outputs and D.rank == 0 else None)
     conv_ms = sum(a.elapsed_time(b) for a, b in ev_pairs)
     e2e_ms = None
     if not args.no_e2e:
@@ -685,7 +730,7 @@ def stack_workload(args, D):
             "conv_s_per_step": conv_ms * 1e-3 / args.steps, "conv_bytes": conv_bytes,
             "conv_words": conv_words, "n_conv": len(ev_pairs), "conv_share": conv_ms / total_ms,
             "in_bytes": sum(x.numel() * 4 for x in host_in),
-            "out_bytes": sum(x.numel() * 4 for x in host_out)}
+            "out_bytes": sum(x.numel() * 4 for x in host_out), "outputs": outputs}
 
 
 SWEEP_MN = (256, 512, 1024, 2048, 4096)
@@ -730,7 +775,7 @@ def bgemm_sweep(args, D):
                     for _ in range(3):
                         gemm(A, out)
                     ts = []
-                    for _ in range(7):
+                    for _ in range(args.steps):
                         flush.zero_()                       # L2 flush between timed launches
                         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                         e0.record(); gemm(A, out); e1.record()
@@ -770,7 +815,7 @@ def main_b200(args):
             best = max(rows, key=lambda r: r["binary_TOPS"])
             best_hbm = max(rows, key=lambda r: r["hbm_frac"])
             emit({"metric": METRIC["bgemm_sweep"], "value": best["binary_TOPS"],
-                  "unit": "binary TOPS", "n_gpus": D.world, "steps": 7, "warmup": 3,
+                  "unit": "binary TOPS", "n_gpus": D.world, "steps": args.steps, "warmup": 3,
                   "ms_per_step": best["ms"], "higher_is_better": True,
                   "scaling": "strong", "vs_baseline": None,
                   "dtype": "s8 x s8 -> s32 on tcgen05 kind::i8 (== xor-popcount, bit-exact)",
@@ -797,12 +842,12 @@ def main_b200(args):
         if extras:
             parity = parity_check(model_bytes, input_type)
         r = graph_workload(D, args.workload, B, input_type, K, args.warmup, want_e2e=not args.no_e2e,
-                           model_bytes=model_bytes)
+                           model_bytes=model_bytes, want_outputs=bool(args.dump_outputs) and D.rank == 0)
     launches = int(D.sum(r["launches"]))
     multi_extra = None
     if D.world > 1 and args.workload == "quicknet" and not args.no_extras:
         # BASELINE.json configs[2] next to configs[1]: QuickNetLarge, batch 128 per GPU (1024 at N = 8)
-        multi_extra = graph_workload(D, "quicknet_large", 128, input_type, max(5, min(K, 10)), 3,
+        multi_extra = graph_workload(D, "quicknet_large", 128, input_type, K, 3,
                                      want_e2e=not args.no_e2e)
     if D.rank != 0:
         if D.world > 1:
@@ -864,23 +909,22 @@ def main_b200(args):
         line["parity_checked"] = True
         line["parity"] = parity
     if extras:
-        Kx = max(5, min(K, 10))
         other_in = "float32" if input_type == "int8" else "int8"
-        f = graph_workload(D, args.workload, B, other_in, Kx, 3, want_e2e=not args.no_e2e,
+        f = graph_workload(D, args.workload, B, other_in, K, 3, want_e2e=not args.no_e2e,
                            want_profile=False)
         line[f"{'f32' if other_in == 'float32' else 'int8'}_input"] = {
-            "value": B / (f["total_ms"] / Kx * 1e-3), "ms_per_step": f["total_ms"] / Kx,
-            "e2e": {"value": B / (f["e2e_ms"] / Kx * 1e-3), "h2d_bytes_per_step": f["in_bytes"],
+            "value": B / (f["total_ms"] / K * 1e-3), "ms_per_step": f["total_ms"] / K,
+            "e2e": {"value": B / (f["e2e_ms"] / K * 1e-3), "h2d_bytes_per_step": f["in_bytes"],
                     "d2h_bytes_per_step": f["out_bytes"]} if f["e2e_ms"] else None,
-            "unit": "images/s", "steps": Kx,
+            "unit": "images/s", "steps": K,
             "note": "the same graph with the other input type, same run"}
         line["legacy_paths"] = {}
         for name, env in (("mma_sync_int8", {"LCE_B200_BCONV_TC": "0"}),
                           ("xor_popc", {"LCE_B200_BCONV_TC": "0", "LCE_B200_BCONV_IMMA": "0"})):
-            x = graph_workload(D, args.workload, B, input_type, Kx, 3, want_e2e=False,
+            x = graph_workload(D, args.workload, B, input_type, K, 3, want_e2e=False,
                                want_profile=False, model_bytes=model_bytes, env=env)
-            line["legacy_paths"][name] = {"value": B / (x["total_ms"] / Kx * 1e-3), "unit": "images/s",
-                                          "ms_per_step": x["total_ms"] / Kx, "env": env}
+            line["legacy_paths"][name] = {"value": B / (x["total_ms"] / K * 1e-3), "unit": "images/s",
+                                          "ms_per_step": x["total_ms"] / K, "env": env}
         line["legacy_paths"]["note"] = ("same graph, same run, every LceBconv2d on the round-1 kernels: "
                                         "int8 mma.sync (lce_b200_imma.cuh) and the XOR + POPC kernel "
                                         "north_star describes (lce_b200_kernels.cuh)")
@@ -888,28 +932,29 @@ def main_b200(args):
         for wl, b in (("birealnet18", 512), ("quicknet_large", 128)):
             if wl == args.workload:
                 continue
-            o = graph_workload(D, wl, b, input_type, Kx, 3, want_e2e=not args.no_e2e)
+            o = graph_workload(D, wl, b, input_type, K, 3, want_e2e=not args.no_e2e)
             ach = o["conv_bytes"] / o["conv_s_per_step"] / 1e9
             line["other_configs"][wl] = {
-                "batch": b, "value": b / (o["total_ms"] / Kx * 1e-3), "unit": "images/s",
-                "ms_per_step": o["total_ms"] / Kx, "steps": Kx,
-                "e2e": b / (o["e2e_ms"] / Kx * 1e-3) if o["e2e_ms"] else None,
+                "batch": b, "value": b / (o["total_ms"] / K * 1e-3), "unit": "images/s",
+                "ms_per_step": o["total_ms"] / K, "steps": K,
+                "e2e": b / (o["e2e_ms"] / K * 1e-3) if o["e2e_ms"] else None,
                 "roofline": {"bound": "hbm", "achieved": ach, "peak": hbm_peak, "unit": "GB/s",
                              "frac": ach / hbm_peak, "share_of_step": o["conv_share"]},
                 "by_op_ms_per_step": o["by_op_ms_per_step"]}
     if multi_extra is not None:
-        Kx = max(5, min(K, 10))
         o = multi_extra
         ach = o["conv_bytes"] / o["conv_s_per_step"] / 1e9
         line["other_configs"] = {"quicknet_large": {
             "batch_per_gpu": 128, "global_batch": 128 * D.world,
-            "value": 128 * D.world / (o["total_ms"] / Kx * 1e-3), "unit": "images/s",
-            "ms_per_step": o["total_ms"] / Kx, "steps": Kx,
-            "e2e": 128 * D.world / (o["e2e_ms"] / Kx * 1e-3) if o["e2e_ms"] else None,
+            "value": 128 * D.world / (o["total_ms"] / K * 1e-3), "unit": "images/s",
+            "ms_per_step": o["total_ms"] / K, "steps": K,
+            "e2e": 128 * D.world / (o["e2e_ms"] / K * 1e-3) if o["e2e_ms"] else None,
             "roofline": {"bound": "hbm", "achieved": ach, "peak": hbm_peak, "unit": "GB/s",
                          "frac": ach / hbm_peak, "share_of_step": o["conv_share"]}}}
     if not args.no_cpu_baseline and D.world == 1:
         line["cpu_baseline"] = cpu_baseline_subprocess(args.workload, B, input_type or "float32")
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, r["outputs"])
     emit(line)
     if D.world > 1:
         D.dist.destroy_process_group()

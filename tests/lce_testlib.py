@@ -10,6 +10,7 @@ scale = 1/n with n in [1,20] and zero point in [-20,20] (tests/utils.h:60-65).
 from __future__ import annotations
 
 import ctypes as C
+import json
 import os
 import subprocess
 from dataclasses import dataclass, field
@@ -315,6 +316,104 @@ def make_bconv_case(seed, batch, in_h, in_w, cin, fh, fw, cout, groups=1,
         thr = compute_thresholds(cin_pg, fh, fw, mul, bias, activation)
     return BconvCase(desc, pack_signs(x), pack_signs(w), mul, bias, thr,
                      {"seed": seed})
+
+
+def golden_op_cases():
+    """Yield (section, index entry, input) for the LceQuantize / LceDequantize / LceBMaxPool2d
+    golden vectors in the order tests/golden/make_golden.py minted them. The inputs are drawn
+    from one seeded stream, so only the reference's outputs are stored; this order is part of
+    the golden data. Grids: bitpack_test.cc:102-109, quantization_test.cc:121-130,
+    bmaxpool_test.cc:204-218 (pruned)."""
+    rng = np.random.default_rng(7)
+    # the special values the bit semantics hinge on (SURVEY 9.3-2)
+    specials = np.array([-0.0, 0.0, np.nan, -np.nan, -1e-30, -1e-45, 1e-45, -np.inf, np.inf],
+                        np.float32)
+    n = 0
+    for rows in (1, 2, 3, 8, 10, 15, 64):
+        for cols in (1, 3, 16, 32, 33, 63, 64, 128):
+            xf = rng.uniform(-1.5, 1.5, (rows, cols)).astype(np.float32)
+            flat = xf.reshape(-1)
+            flat[: min(flat.size, specials.size)] = specials[: flat.size]
+            yield "quantize", {"key": f"q_f32_{n}", "type": "f32", "zero_point": 0}, xf
+            for zp in (-1000, -1, 0, 23, 127, 128):
+                xi = rng.integers(-128, 128, (rows, cols), dtype=np.int8)
+                yield "quantize", {"key": f"q_i8_{n}_{zp}", "type": "i8", "zero_point": zp}, xi
+            xb = rng.integers(0, 2, (rows, cols), dtype=np.uint8).astype(np.bool_)
+            yield "quantize", {"key": f"q_b_{n}", "type": "bool", "zero_point": 1}, xb
+            n += 1
+    for n, (shape, ch) in enumerate([((1, 4, 4), 1), ((2, 3, 3), 31), ((1, 5, 2), 32),
+                                     ((1, 2, 2), 33), ((3, 1, 1), 64), ((1, 3, 3), 68),
+                                     ((1, 2, 3), 130), ((1, 1, 2), 200)]):
+        packed = rng.integers(-2**31, 2**31, shape + (cdiv(ch, 32),),
+                              dtype=np.int64).astype(np.int32)
+        for t, scale, zp in ((T_FLOAT, 1.0, 0), (T_BOOL, 1.0, 0), (T_INT8, 1.0, 0),
+                             (T_INT8, 0.05, 3), (T_INT8, 0.007, -100), (T_INT8, 0.3, 127)):
+            yield "dequantize", {"key": f"dq_{n}_{t}_{zp}", "channels": ch, "type": t,
+                                 "scale": scale, "zero_point": zp}, packed
+    n = 0
+    for (b, h, w, ch) in ((1, 7, 7, 1), (4, 8, 5, 2), (1, 12, 9, 3), (2, 56, 56, 2)):
+        for (fh, fw) in ((1, 1), (2, 2), (3, 3), (2, 3)):
+            for (sh, sw) in ((1, 1), (2, 2), (2, 3)):
+                for pad in (PADDING_SAME, PADDING_VALID):
+                    if pad == PADDING_VALID and (fh > h or fw > w):
+                        continue
+                    x = rng.integers(-2**31, 2**31, (b, h, w, ch), dtype=np.int64).astype(np.int32)
+                    yield "bmaxpool", {"key": f"mp_{n}",
+                                       "desc": [b, h, w, ch, fh, fw, sh, sw, pad]}, x
+                    n += 1
+
+
+def random_walk_cases():
+    """Yield (n, case, optimised) for the seeded 300-step walk over LceBconv2d parameters that
+    tests/test_oracle.py checks against the reference; `optimised` is True where the optimised
+    kernels (kind 1) accept the case. Drawn from one stream: the order is part of the golden data."""
+    rng = np.random.default_rng(99)
+    for n in range(300):
+        c = int(rng.choice([4, 32, 64, 96, 128, 192, 256]))
+        g = int(rng.choice([1, 2])) if c % 64 == 0 else 1
+        co = int(rng.choice([1, 2, 4, 6, 32, 34, 64])) * g
+        fh, fw = int(rng.integers(1, 4)), int(rng.integers(1, 4))
+        h, w = int(rng.integers(3, 10)), int(rng.integers(3, 10))
+        st = (int(rng.integers(1, 3)), int(rng.integers(1, 4)))
+        dl = (int(rng.integers(1, 3)), int(rng.integers(1, 3)))
+        pad, pv = [(PADDING_VALID, 1), (PADDING_SAME, 0), (PADDING_SAME, 1)][n % 3]
+        if pad == PADDING_VALID and ((fh - 1) * dl[0] + 1 > h or (fw - 1) * dl[1] + 1 > w):
+            dl = (1, 1)
+        if pad == PADDING_SAME and pv == 0 and c % 2:
+            pv = 1
+        ot = [OUT_FLOAT, OUT_INT8, OUT_BITPACKED][n % 3 if n % 2 else (n // 2) % 3]
+        act = int(rng.integers(0, 4))
+        case = make_bconv_case(n, int(rng.integers(1, 3)), h, w, c, fh, fw, co, g,
+                               st, dl, pad, pv, act, ot)
+        if ot == OUT_BITPACKED and act not in (ACT_NONE, ACT_RELU):
+            continue
+        optimised = g == 1 and not (pad == PADDING_SAME and pv == 0 and
+                                    (ot != OUT_FLOAT or act != ACT_NONE))
+        yield n, case, optimised
+
+
+GOLDEN_DIR = os.path.join(REPO, "tests", "golden")
+# The reference's outputs, split so that no committed file exceeds 1 MB.
+GOLDEN_FILES = {"bconv": "lce_golden_bconv.npz", "ops": "lce_golden_ops.npz"}
+
+
+def load_golden():
+    """(index, arrays) of the golden vectors: the reference's outputs under their keys, and the
+    regenerated input of every quantize / dequantize / bmaxpool vector under key + "_in"."""
+    with open(os.path.join(GOLDEN_DIR, "lce_golden.json")) as f:
+        index = json.load(f)["index"]
+    arrays = {}
+    for name in GOLDEN_FILES.values():
+        with np.load(os.path.join(GOLDEN_DIR, name)) as z:
+            arrays.update((k, z[k]) for k in z.files)
+    arrays.update((e["key"] + "_in", x) for _, e, x in golden_op_cases())
+    return index, arrays
+
+
+def load_random_walk():
+    """{str(n): {"kind0": sha256, "kind1": sha256 (where optimised)}} of random_walk_cases()."""
+    with open(os.path.join(GOLDEN_DIR, "lce_random_walk.json")) as f:
+        return json.load(f)["cases"]
 
 
 def desc_to_dict(d: BconvDesc):

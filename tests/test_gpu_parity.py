@@ -4,8 +4,6 @@ seeded inputs and against the committed golden vectors minted from the reference
 Bar: bit-exact for bitpacked / int8 / int32 results AND for float results (the
 epilogue reproduces the reference's two-rounding multiply-add)."""
 import hashlib
-import json
-import os
 
 import numpy as np
 import pytest
@@ -14,8 +12,6 @@ import torch
 import lce_testlib as L
 
 pytestmark = pytest.mark.gpu
-
-GOLD_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
@@ -27,9 +23,7 @@ def capi():
 
 @pytest.fixture(scope="module")
 def golden():
-    with open(os.path.join(GOLD_DIR, "lce_golden.json")) as f:
-        index = json.load(f)["index"]
-    return index, np.load(os.path.join(GOLD_DIR, "lce_golden.npz"))
+    return L.load_golden()
 
 
 def dev(a):

@@ -1,25 +1,19 @@
 """CPU tests of the checker itself: the plain-C oracle (oracle/lce_oracle.c) is
 pinned against (1) the known-answer vectors in the reference's own tests, (2) the
 committed golden vectors minted from the compiled reference headers
-(tests/golden/make_golden.py), and (3) the compiled reference live when
-oracle/_ref/liblce_ref.so is present (build container only)."""
+(tests/golden/make_golden.py), and (3) the reference's results on a 300-case random walk
+(stored digests; live as well when oracle/_ref/liblce_ref.so is built)."""
 import hashlib
-import json
-import os
 
 import numpy as np
 import pytest
 
 import lce_testlib as L
 
-GOLD_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
 
 @pytest.fixture(scope="module")
 def golden():
-    with open(os.path.join(GOLD_DIR, "lce_golden.json")) as f:
-        index = json.load(f)["index"]
-    return index, np.load(os.path.join(GOLD_DIR, "lce_golden.npz"))
+    return L.load_golden()
 
 
 def case_from_spec(entry):
@@ -225,40 +219,27 @@ def test_golden_quantize_dequantize_bmaxpool(golden):
         assert np.array_equal(L.bmaxpool(d, arrays[e["key"] + "_in"]), arrays[e["key"]]), e
 
 
-# ---- (3) live against the compiled reference (build container only) ------- #
-@pytest.mark.skipif(L.load_ref() is None, reason="oracle/_ref not built here")
+# ---- (3) against the compiled reference: stored digests, and live where oracle/_ref exists -- #
 def test_live_reference_random_walk():
-    rng = np.random.default_rng(99)
-    for n in range(300):
-        c = int(rng.choice([4, 32, 64, 96, 128, 192, 256]))
-        g = int(rng.choice([1, 2])) if c % 64 == 0 else 1
-        co = int(rng.choice([1, 2, 4, 6, 32, 34, 64])) * g
-        fh, fw = int(rng.integers(1, 4)), int(rng.integers(1, 4))
-        h, w = int(rng.integers(3, 10)), int(rng.integers(3, 10))
-        st = (int(rng.integers(1, 3)), int(rng.integers(1, 4)))
-        dl = (int(rng.integers(1, 3)), int(rng.integers(1, 3)))
-        pad, pv = [(L.PADDING_VALID, 1), (L.PADDING_SAME, 0), (L.PADDING_SAME, 1)][n % 3]
-        if pad == L.PADDING_VALID and ((fh - 1) * dl[0] + 1 > h or (fw - 1) * dl[1] + 1 > w):
-            dl = (1, 1)
-        if pad == L.PADDING_SAME and pv == 0 and c % 2:
-            pv = 1
-        ot = [L.OUT_FLOAT, L.OUT_INT8, L.OUT_BITPACKED][n % 3 if n % 2 else (n // 2) % 3]
-        act = int(rng.integers(0, 4))
-        case = L.make_bconv_case(n, int(rng.integers(1, 3)), h, w, c, fh, fw, co, g,
-                                 st, dl, pad, pv, act, ot)
-        if ot == L.OUT_BITPACKED and act not in (L.ACT_NONE, L.ACT_RELU):
-            continue
-        a = L.bconv2d(case.desc, case.inp, case.filt, case.mul, case.bias, case.thr)
-        b = L.bconv2d(case.desc, case.inp, case.filt, case.mul, case.bias, case.thr,
-                      impl="ref", kind=0)
-        assert np.array_equal(a.view(np.uint8), b.view(np.uint8)), L.desc_to_dict(case.desc)
-        # the optimised kernels (indirect BGEMM + float zero-padding correction) where legal
-        if g == 1 and not (pad == L.PADDING_SAME and pv == 0 and
-                           (ot != L.OUT_FLOAT or act != L.ACT_NONE)):
-            a1 = L.bconv2d(case.desc, case.inp, case.filt, case.mul, case.bias, case.thr, kind=1)
-            b1 = L.bconv2d(case.desc, case.inp, case.filt, case.mul, case.bias, case.thr,
-                           impl="ref", kind=1)
-            assert np.array_equal(a1.view(np.uint8), b1.view(np.uint8)), L.desc_to_dict(case.desc)
+    """300 seeded LceBconv2d cases (lce_testlib.random_walk_cases): the oracle's reference-kernel
+    result (kind 0) and, where legal, its optimised-kernel result (kind 1) equal the reference's,
+    held as digests in tests/golden/lce_random_walk.json; with oracle/_ref built, also compared
+    with the compiled reference live."""
+    stored = L.load_random_walk()
+    ref = L.load_ref()
+    seen = 0
+    for n, case, optimised in L.random_walk_cases():
+        e, where = stored[str(n)], L.desc_to_dict(case.desc)
+        args = (case.desc, case.inp, case.filt, case.mul, case.bias, case.thr)
+        for kind in (0, 1) if optimised else (0,):
+            a = L.bconv2d(*args, kind=kind)
+            assert hashlib.sha256(a.tobytes()).hexdigest() == e[f"kind{kind}"], (n, kind, where)
+            if ref is not None:
+                b = L.bconv2d(*args, impl="ref", kind=kind)
+                assert np.array_equal(a.view(np.uint8), b.view(np.uint8)), (n, kind, where)
+        assert optimised == ("kind1" in e), (n, where)
+        seen += 1
+    assert seen == len(stored)
 
 
 def test_oracle_bgemm_equals_1x1_bconv():
