@@ -538,11 +538,10 @@ int tc_launch(GemmCore& c, const lce::ConvKParams& p, cudaStream_t s) {
   }
 }
 
+}  // namespace
 // fp32 pointwise convolution on the tensor cores (lce_b200_pw.cuh), called by the CONV_2D builtin
 // (lce_b200_builtins.cu). 0 = launched, -1 = shape not eligible (the caller's FMA kernels take
 // it), > 0 = error.
-std::atomic<uint64_t> g_pw_launches{0};
-}  // namespace
 namespace lce_b200_internal {
 int pw_tf32_conv(const float* in, const float* filter, const float* bias, float* out, int32_t* packed, long long M, int N,
                  int K, int act, int pairs_ok, void* stream) {
@@ -626,10 +625,8 @@ int pw_tf32_conv(const float* in, const float* filter, const float* bias, float*
       fprintf(stderr, "[pw prof]  %-7s w%-2d total=%lld  c1=%lld c2=%lld c3=%lld c4=%lld n=%lld\n", names[w], w, h[w * 8], h[w * 8 + 1],
               h[w * 8 + 2], h[w * 8 + 3], h[w * 8 + 4], h[w * 8 + 5]);
   }
-  g_pw_launches.fetch_add(1, std::memory_order_relaxed);
   return launch_check("pw_tf32_kernel");
 }
-uint64_t pw_tf32_launches() { return g_pw_launches.load(); }
 // CONV_2D 7x7 / stride 2 / 3 -> 64 (Bi-RealNet's stem) on tcgen05 kind::tf32 (lce_b200_pw.cuh):
 // 0 = launched, -1 = not this shape, > 0 = error.
 int stem7_tf32_conv(const float* in, const float* filter, const float* bias, float* out, int B, int H, int W, int OH, int OW,
@@ -660,7 +657,6 @@ int stem7_tf32_conv(const float* in, const float* filter, const float* bias, flo
     CUDA_OK(cudaFuncSetAttribute(P::stem7_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(P::kS7Smem)));
   const int grid = static_cast<int>(std::min<long long>(m_tiles, num_sms()));
   P::stem7_tf32_kernel<<<grid, P::kS7Threads, P::kS7Smem, static_cast<cudaStream_t>(stream)>>>(tm_out, p);
-  g_pw_launches.fetch_add(1, std::memory_order_relaxed);
   return launch_check("stem7_tf32_kernel");
 }
 }  // namespace lce_b200_internal

@@ -7,6 +7,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cfloat>
 #include <climits>
 #include <cstdint>
@@ -63,6 +64,17 @@ int grid_for(long long n, int per_block, int max_blocks = 148 * 32) {
 struct ConvGeom {
   int B, H, W, Cin, KH, KW, Cout, sh, sw, dh, dw, ph, pw, OH, OW, act;
 };
+
+// successful launches per fp32 convolution kernel (lce_b200_f32_conv_path_counts)
+enum ConvPath { kPathPwTf32, kPathStem7, kPathDirect16, kPathGemmSmallM, kPathGemm128, kPathIgemm8x8, kPathIgemm8x4,
+                kPathGemm, kConvPaths };
+std::atomic<uint64_t> g_conv_path[kConvPaths] = {};
+void count_path(ConvPath p) { g_conv_path[p].fetch_add(1, std::memory_order_relaxed); }
+int launched(ConvPath p, const char* what) {
+  const int rc = launch_check(what);
+  if (rc == 0) count_path(p);
+  return rc;
+}
 
 // ---- small-K direct convolution (stem 3x3x3->16, 16->64 pointwise: K <= 32) --------
 // One thread = one output pixel x 16 consecutive output channels; consecutive lanes
@@ -1481,6 +1493,7 @@ static int conv2d_impl(const lce_f32_conv_desc* d, const float* in, const float*
     const int rc = lce_b200_internal::pw_tf32_conv(in, filter, bias, out, pk, M, g.Cout, K, g.act,
                                                    ((static_cast<long long>(g.OH) * g.OW) & 1) == 0, stream);
     if (rc >= 0) {
+      if (rc == 0) count_path(kPathPwTf32);
       if (rc == 0 && pk) *packed_done = true;
       return rc;
     }
@@ -1488,6 +1501,7 @@ static int conv2d_impl(const lce_f32_conv_desc* d, const float* in, const float*
   if (g.KH == 7 && g.KW == 7 && g.Cin == 3 && g.Cout == 64 && g.sh == 2 && g.sw == 2 && g.dh == 1 && g.dw == 1) {
     const int rc = lce_b200_internal::stem7_tf32_conv(in, filter, bias, out, g.B, g.H, g.W, g.OH, g.OW, g.ph, g.pw, g.act,
                                                       stream);
+    if (rc == 0) count_path(kPathStem7);
     if (rc >= 0) return rc;
   }
   const int Gd = (g.Cout + 15) / 16;
@@ -1549,7 +1563,7 @@ static int conv2d_impl(const lce_f32_conv_desc* d, const float* in, const float*
       LCE_DIRECT(0, 0, 0, 4);
     }
 #undef LCE_DIRECT
-    return launch_check("conv_direct16_kernel");
+    return launched(kPathDirect16, "conv_direct16_kernel");
   }
   const bool plain = g.KH == 1 && g.KW == 1 && g.sh == 1 && g.sw == 1 && (K & 3) == 0 &&
                      !((uintptr_t)in & 15) && !((uintptr_t)filter & 15) && !((uintptr_t)out & 15);
@@ -1557,7 +1571,7 @@ static int conv2d_impl(const lce_f32_conv_desc* d, const float* in, const float*
     dim3 sgrid(static_cast<unsigned>((M + kSM_ - 1) / kSM_), (g.Cout + kSN_ - 1) / kSN_);
     gemm_small_m_kernel<<<sgrid, 256, 0, as_stream(stream)>>>(in, filter, bias, out, M, g.Cout, K,
                                                               g.act);
-    return launch_check("gemm_small_m_kernel");
+    return launched(kPathGemmSmallM, "gemm_small_m_kernel");
   }
   if (plain) {
     dim3 grid(static_cast<unsigned>((M + kPM - 1) / kPM), (g.Cout + kPN - 1) / kPN);
@@ -1565,25 +1579,41 @@ static int conv2d_impl(const lce_f32_conv_desc* d, const float* in, const float*
     if (pk) *packed_done = true;
     conv_gemm128_kernel<<<grid, 256, 0, as_stream(stream)>>>(in, filter, bias, out, M, g.Cout, K,
                                                              g.act, pk);
-    return launch_check("conv_gemm128_kernel");
+    return launched(kPathGemm128, "conv_gemm128_kernel");
   }
   if (K <= kIKMax && static_cast<long long>(g.H) * g.W * g.Cin < (1LL << 31)) {
     dim3 igrid(static_cast<unsigned>((M + kIM - 1) / kIM), (g.Cout + kIN - 1) / kIN);
     const size_t ksmem = static_cast<size_t>((K + kIK - 1) / kIK * kIK) * 2 * sizeof(int);
+    // 25,600 B of static tiles plus a k-table of up to 32 KB: above K = 2944 a block needs more than
+    // the default 48 KB, so both kernels opt in to the table's maximum (once per device)
+    static bool attr[64] = {};   // the attribute is per device
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64 || !attr[dev]) {
+      constexpr int kTabMax = kIKMax * 2 * sizeof(int);
+      if (cudaFuncSetAttribute(conv_igemm8x8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTabMax) != cudaSuccess ||
+          cudaFuncSetAttribute(conv_igemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTabMax) != cudaSuccess)
+        return fail("conv igemm: cannot raise the shared-memory limit");
+      if (dev >= 0 && dev < 64) attr[dev] = true;
+    }
     static const bool use8x4 = [] {
       const char* e = getenv("LCE_B200_IGEMM_8X4");
       return e && e[0] == '1';
     }();
     if (use8x4) {
       conv_igemm_kernel<<<igrid, 256, ksmem, as_stream(stream)>>>(in, filter, bias, out, g, M);
-      return launch_check("conv_igemm_kernel");
+      return launched(kPathIgemm8x4, "conv_igemm_kernel");
     }
     conv_igemm8x8_kernel<<<igrid, 128, ksmem, as_stream(stream)>>>(in, filter, bias, out, g, M);
-    return launch_check("conv_igemm8x8_kernel");
+    return launched(kPathIgemm8x8, "conv_igemm8x8_kernel");
   }
   dim3 grid(static_cast<unsigned>((M + kGM - 1) / kGM), (g.Cout + kGN - 1) / kGN);
   conv_gemm_kernel<<<grid, 256, 0, as_stream(stream)>>>(in, filter, bias, out, g, M);
-  return launch_check("conv_gemm_kernel");
+  return launched(kPathGemm, "conv_gemm_kernel");
+}
+
+void lce_b200_f32_conv_path_counts(uint64_t out[8]) {
+  for (int i = 0; i < kConvPaths; ++i) out[i] = g_conv_path[i].load();
 }
 
 int lce_b200_f32_conv2d(const lce_f32_conv_desc* d, const float* in, const float* filter,
@@ -1634,8 +1664,10 @@ int lce_b200_f32_depthwise_conv2d(const lce_f32_conv_desc* d, const float* in,
 int lce_b200_f32_pool_out_shape(const lce_f32_pool_desc* d, int* out_h, int* out_w) {
   if (d->filter_h < 1 || d->filter_w < 1 || d->stride_h < 1 || d->stride_w < 1)
     return fail("pool: bad parameters");
-  *out_h = out_size(d->padding, d->in_h, d->filter_h, d->stride_h, 1);
-  *out_w = out_size(d->padding, d->in_w, d->filter_w, d->stride_w, 1);
+  // VALID with a filter larger than the input has no output (as in make_geom): two negative
+  // extents must not multiply into a positive element count
+  *out_h = std::max(0, out_size(d->padding, d->in_h, d->filter_h, d->stride_h, 1));
+  *out_w = std::max(0, out_size(d->padding, d->in_w, d->filter_w, d->stride_w, 1));
   return 0;
 }
 

@@ -45,6 +45,11 @@ int lce_b200_f32_conv2d(const lce_f32_conv_desc* d, const float* in_dev, const f
 int lce_b200_f32_conv2d_packed(const lce_f32_conv_desc* d, const float* in_dev,
                                const float* filter_dev, const float* bias_dev, float* out_dev,
                                int32_t* packed_out_dev, void* stream);
+/* Diagnostics: successful launches so far of each convolution kernel conv2d(_packed) chooses from:
+ * [0] tcgen05 tf32 pointwise, [1] tcgen05 tf32 7x7 stem, [2] direct (K <= 32), [3] small-M GEMM,
+ * [4] 128x128 GEMM, [5] implicit GEMM 8x8, [6] implicit GEMM 8x4 (LCE_B200_IGEMM_8X4=1),
+ * [7] implicit GEMM for K > 4096. */
+void lce_b200_f32_conv_path_counts(uint64_t out[8]);
 /* depth_multiplier 1; filter [1, fh, fw, C]; d->out_c == d->in_c */
 int lce_b200_f32_depthwise_conv2d(const lce_f32_conv_desc* d, const float* in_dev,
                                   const float* filter_dev, const float* bias_dev,

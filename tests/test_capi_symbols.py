@@ -66,6 +66,26 @@ def test_shape_inference_matches_oracle(lib):
         assert tuple(x.value for x in o) == want
 
 
+def test_float_shape_inference_matches_tflite(lib):
+    """lce_b200_f32_conv_out_shape / _pool_out_shape against TFLite's rule: SAME out = ceil(in / s),
+    VALID out = max(floor((in - (k - 1) d - 1) / s) + 1, 0)."""
+    from test_gpu_float_kernels import ConvDesc, PoolDesc, tfl_out_pad
+    oh, ow = C.c_int(), C.c_int()
+    for n in (1, 2, 3, 4, 7, 8, 56):
+        for k in (1, 2, 3, 5, 7):
+            for s in (1, 2, 3):
+                for d in (1, 2):
+                    for pad in (0, 1):
+                        want = tfl_out_pad(pad, n, k, s, d)[0]
+                        desc = ConvDesc(2, n, n + 1, 3, k, 1, 4, s, 1, d, 1, pad, 0)
+                        assert lib.lce_b200_f32_conv_out_shape(C.byref(desc), C.byref(oh), C.byref(ow)) == 0
+                        assert (oh.value, ow.value) == (want, tfl_out_pad(pad, n + 1, 1, 1)[0]), (n, k, s, d, pad)
+                        if d == 1:
+                            p = PoolDesc(2, n + 1, n, 4, 1, k, 1, s, pad, 0)
+                            assert lib.lce_b200_f32_pool_out_shape(C.byref(p), C.byref(oh), C.byref(ow)) == 0
+                            assert (oh.value, ow.value) == (tfl_out_pad(pad, n + 1, 1, 1)[0], want), (n, k, s, pad)
+
+
 def test_no_cpu_fallback_without_device(lib):
     import torch
     if torch.cuda.is_available():
@@ -80,6 +100,6 @@ def test_no_cpu_fallback_without_device(lib):
 
 def test_builtin_kernels_header_symbols_are_exported(lib):
     names = declared_symbols("lce_b200_builtins.h")
-    assert len(names) == 17
+    assert len(names) == 18
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/lce_b200_builtins.h but not exported"
